@@ -24,7 +24,8 @@ extern "C" {
 #endif
 
 enum { VDB_OK = 0, VDB_ERR_INVALID = 1, VDB_ERR_CUDA = 2, VDB_ERR_UNSUPPORTED = 3 };
-enum { VDB_ACT_NONE = 0, VDB_ACT_SILU = 1, VDB_ACT_GELU = 2, VDB_ACT_QUICK_GELU = 3, VDB_ACT_GEGLU = 4 };
+enum { VDB_ACT_NONE = 0, VDB_ACT_SILU = 1, VDB_ACT_GELU = 2, VDB_ACT_QUICK_GELU = 3, VDB_ACT_GEGLU = 4,
+       VDB_ACT_GELU_TANH = 5 /* GPT-2's tanh-form GELU, optimus_gpt2.py:99-100 */ };
 
 /* ---- library state ------------------------------------------------------------------------- */
 const char* vdb_version(void);
@@ -228,6 +229,32 @@ int vdb_pack_geglu(const float* w, const float* b, int n2, int K, void* w_out, f
 /* CrossAttention.to_q / to_k / to_v weight [H*d, K] (attention.py:152-168) -> [H*dpad, K] with zero rows after each head's d
  * rows; dpad = vdb_attention_dk_pad(d) for q / k, vdb_attention_dv_pad(d) for v. */
 int vdb_pad_heads(const float* w, int H, int d, int dpad, int K, void* out, void* stream);
+
+/* ---- Optimus GPT-2 text decode with a KV cache — optimus_vae_next.decode / sample_single_sequence_conditional
+ *      (lib/model_zoo/optimus.py:662-688, 745-763) on GPT2ForLatentConnector_XX (optimus_models/optimus_gpt2.py:813-1112).
+ *      The reference re-runs the whole prefix per token; these kernels keep a per-layer bf16 KV cache [n, H, 32, 64] instead.
+ *      `step` is a device int: the index t (0 = <BOS>) of the token being processed, so one captured graph serves every step
+ *      (advance it with vdb_add_int). Sequences hold at most 30 tokens (max_length of optimus.py:751). -------------------- */
+/* Single-query attention of token t (Attention.forward / _attn, optimus_gpt2.py:151-209), d_head 64, any H:
+ * appends k, v of qkv[row] = [q | k | v] (each H*64, the c_attn output) at slot t of kcache / vcache, then attends over
+ * key 0 = the latent memory mem[row, h*64 ..] (a layer's slice of linear(z), used as past key AND value, :887-893) and the
+ * cached tokens 0..t; out[row, h*64 ..] = softmax(q k^T * scale) v (fp32 softmax).  ldqkv, ldmem multiples of 8. */
+int vdb_kv_decode_attention(const void* qkv, long long ldqkv, const void* mem, long long ldmem, void* kcache, void* vcache,
+                            const int* step, int n, int H, float scale, void* out, long long ldo, void* stream);
+/* One CTA per row: p = softmax(logits[row, :V] / *temperature) (fp32, fixed-order sums), token = smallest i with
+ * cumsum(p)[i] > u (torch.multinomial's draw, optimus.py:678, without the top_p = 1.0 filter, which only drops tokens whose
+ * fp32 cumulative sum rounds above 1).  u = uniforms[row * ldu + t] when uniforms != NULL, else Philox4x32-10 keyed by *seed
+ * with counter (row, t).  A row whose token t is eos stays at eos; a token landing at index max_len-1 becomes eos (:680-685).
+ * forced != NULL ([n, ldt] int32): take forced[row, t+1] instead of sampling (teacher forcing).  Writes tokens[row, t+1] and,
+ * when x_next != NULL, x_next[row] = bf16(wte[token] + wpe[t+2] + emb_add[row]) (GPT2Model_XX.forward, :941-951; positions
+ * start at 1 behind the memory slot).  wte bf16 [>= vocab, C], wpe / emb_add fp32. */
+int vdb_sample_tokens(const float* logits, long long ldl, int V, int n, const float* temperature, const int* step,
+                      const unsigned long long* seed, const float* uniforms, int ldu, const int* forced, int eos, int max_len,
+                      int* tokens, int ldt, const void* wte, const float* wpe, const float* emb_add, long long ld_emb, int C,
+                      void* x_next, long long ldx, void* stream);
+/* x[row] = bf16(wte[tokens[row, t]] + wpe[t + pos_offset] + emb_add[row]), t = *step (0 when step == NULL): the <BOS> input. */
+int vdb_token_embed(const int* tokens, int ldt, const int* step, int pos_offset, const void* wte, const float* wpe,
+                    const float* emb_add, long long ld_emb, int n, int C, void* x, long long ldx, void* stream);
 
 #ifdef __cplusplus
 }

@@ -464,5 +464,9 @@ VDB_DEVINL float gelu_fast_f(float x) {
   return fmaf(hx, th, hx);
 }
 VDB_DEVINL float quick_gelu_f(float x) { return __fdividef(x, 1.0f + __expf(-1.702f * x)); }
+// GPT-2's tanh-form GELU, 0.5 x (1 + tanh(sqrt(2/pi) (x + 0.044715 x^3))) (optimus_gpt2.py:99-100), with the accurate tanhf
+VDB_DEVINL float gelu_tanh_f(float x) {
+  return 0.5f * x * (1.0f + tanhf(0.7978845608028654f * (x + 0.044715f * x * x * x)));
+}
 
 }  // namespace vdb

@@ -2,8 +2,9 @@
 
 The reference resolves YAML with `super_cfg` inheritance and MODEL(name) indirection; the values below
 are the resolved results for the shipped configs (configs/model/{vd,openai_unet,autokl,clip}.yaml).
-Text-latent flows (Optimus VAE, 0D data blocks) are outside the hot path: 'vd_four_flow_v1-0' here
-carries the image VAE, both CLIP context encoders, the 2D diffuser and the 0D diffuser's context blocks.
+By default 'vd_four_flow_v1-0' carries the image VAE, both CLIP context encoders, the 2D diffuser and the 0D diffuser's
+context blocks.  VDB_TEXT_FLOWS=1 adds what the text-latent flows (i2t / t2t) need: the 0D diffuser's data blocks and the
+Optimus text VAE's decoder (configs/model/optimus.yaml), registered as vae['text'].
 """
 import copy
 import os
@@ -77,6 +78,26 @@ _BANK = {
     "vd_base": dict(symbol="vd", find_unused_parameters=True, type="vd_v2_0", args=dict(
         beta_linear_start=0.00085, beta_linear_end=0.012, timesteps=1000, use_ema=False)),
 }
+# configs/model/optimus.yaml:43-90, 96-102 with MODEL(...) resolved; only the decoder side is built (the BERT encoder is used
+# by no app.py flow), and the training-only fields (dropouts, summary heads) are left out
+_TEXT_BANK = {
+    "optimus_gpt2_decoder": dict(symbol="optimus", find_unused_parameters=False, type="optimus_gpt2_connector", args=dict(
+        config=dict(hidden_size=768, initializer_range=0.02, latent_size=768, layer_norm_epsilon=1e-05,
+                    max_position_embeddings=1024, n_ctx=1024, n_embd=768, n_head=12, n_layer=12, n_positions=1024,
+                    num_attention_heads=12, num_hidden_layers=12, vocab_size=50260))),
+    "optimus_gpt2_tokenizer": dict(symbol="optimus", find_unused_parameters=False, type="optimus_gpt2_tokenizer", args=dict(
+        do_lower_case=False, max_len=1024, vocab_file="lib/model_zoo/optimus_models/vocab/gpt2-vocab.json",
+        merges_file="lib/model_zoo/optimus_models/vocab/gpt2-merges.txt")),
+}
+_TEXT_BANK["optimus_v1"] = dict(symbol="optimus", find_unused_parameters=False, type="optimus_vae_next", args=dict(
+    decoder=_TEXT_BANK["optimus_gpt2_decoder"], tokenizer_decoder=_TEXT_BANK["optimus_gpt2_tokenizer"],
+    args=dict(latent_size=768)))
+
+
+def _text_flows():
+    return os.environ.get("VDB_TEXT_FLOWS") == "1"
+
+
 for _sfx, _parts in _PARTS.items():
     _BANK["openai_unet_2d_v1" + _sfx] = _unet2d(_parts)
     _BANK["openai_unet_0d_v1" + _sfx] = _unet0d(_parts)
@@ -86,15 +107,19 @@ class model_cfg_bank(object):
     def __call__(self, name):
         if name == "vd_four_flow_v1-0":
             cfg = CfgDict(copy.deepcopy(_BANK["vd_base"]))
+            vaes = [["image", self("autokl_v1")]] + ([["text", self("optimus_v1")]] if _text_flows() else [])
             cfg.args.update(dict(
-                vae_cfg_list=[["image", self("autokl_v1")]],
+                vae_cfg_list=vaes,
                 ctx_cfg_list=[["image", self("clip_image_context_encoder")], ["text", self("clip_text_context_encoder")]],
                 # the 0D (text-latent) diffuser contributes only its context blocks to image sampling; VDB_TEXT_FLOWS=1 builds its
                 # data blocks too (the reference's 'openai_unet_0d_v1_dc': +1.7 G parameters) for the i2t / t2t diffusion
                 diffuser_cfg_list=[["image", self("openai_unet_2d_v1")],
-                                   ["text", self("openai_unet_0d_v1_dc" if os.environ.get("VDB_TEXT_FLOWS") == "1" else "openai_unet_0d_v1_c")]],
+                                   ["text", self("openai_unet_0d_v1_dc" if _text_flows() else "openai_unet_0d_v1_c")]],
                 global_layer_ptr="image", latent_scale_factor={"image": 0.18215}))
             return cfg
+        if _text_flows() and name in _TEXT_BANK:
+            return CfgDict(copy.deepcopy(_TEXT_BANK[name]))
         if name not in _BANK:
-            raise KeyError(f"config '{name}' is outside the B200 hot-path build (have: {sorted(_BANK)} + vd_four_flow_v1-0)")
+            raise KeyError(f"config '{name}' is outside the B200 hot-path build (have: {sorted(_BANK)} + vd_four_flow_v1-0; "
+                           "VDB_TEXT_FLOWS=1 adds the Optimus text VAE)")
         return CfgDict(copy.deepcopy(_BANK[name]))

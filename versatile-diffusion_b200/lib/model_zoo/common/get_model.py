@@ -6,7 +6,8 @@ import torch
 
 from ...log_service import print_log
 
-_TYPE_TO_MODULE = (("autoencoderkl", "autokl"), ("clip", "clip"), ("vd", "vd"), ("openai_unet", "openaimodel"))
+_TYPE_TO_MODULE = (("autoencoderkl", "autokl"), ("clip", "clip"), ("vd", "vd"), ("openai_unet", "openaimodel"),
+                   ("optimus", "optimus"))
 
 
 class _Registry(object):

@@ -63,6 +63,9 @@ SIGNATURES = {
     "vdb_pack_conv_weight": (i, [p, i, i, i, i, p, ll, ll, p]),
     "vdb_pack_geglu": (i, [p, p, i, i, p, p, p]),
     "vdb_pad_heads": (i, [p, i, i, i, i, p, p]),
+    "vdb_kv_decode_attention": (i, [p, ll, p, ll, p, p, p, i, i, f, p, ll, p]),
+    "vdb_sample_tokens": (i, [p, ll, i, i, p, p, p, p, i, p, i, i, p, i, p, p, p, ll, i, p, ll, p]),
+    "vdb_token_embed": (i, [p, i, p, i, p, p, p, ll, i, i, p, ll, p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -12,7 +12,7 @@ import torch
 
 from ._lib import lib, check
 
-ACT_NONE, ACT_SILU, ACT_GELU, ACT_QUICK_GELU, ACT_GEGLU = 0, 1, 2, 3, 4
+ACT_NONE, ACT_SILU, ACT_GELU, ACT_QUICK_GELU, ACT_GEGLU, ACT_GELU_TANH = 0, 1, 2, 3, 4, 5
 BF16 = torch.bfloat16
 
 
@@ -642,4 +642,51 @@ def scale_by_row_norm(z, L, idx=None, row_scale=None):
     B, Lp, C = z.shape
     out = torch.empty((B, L, C), dtype=torch.float32, device=z.device)
     check(lib.vdb_scale_by_row_norm(_ptr(z), _ptr(idx), _ptr(row_scale), B, L, Lp, C, _ptr(out), _stream()), "scale_by_row_norm")
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
+# Optimus GPT-2 text decode (optimus.py:662-688): KV-cache attention, on-device sampling, <BOS> embedding
+# ------------------------------------------------------------------------------------------------
+def kv_decode_attention(qkv, mem, kcache, vcache, step, H, out, scale=0.125):
+    """qkv [n, >=3*H*64] bf16 (row-strided ok), mem [n, >=H*64] bf16 view of this layer's memory slot, caches bf16
+    [n, H, 32, 64], step int32 [1] device counter; writes out [n, H*64] bf16."""
+    _need(qkv, BF16, "qkv", True); _need(mem, BF16, "mem", True); _need(kcache, BF16, "kcache"); _need(vcache, BF16, "vcache")
+    _need(step, torch.int32, "step"); _need(out, BF16, "out", True)
+    n = qkv.shape[0]
+    assert kcache.numel() >= n * H * 32 * 64 and vcache.numel() >= n * H * 32 * 64
+    check(lib.vdb_kv_decode_attention(_ptr(qkv), qkv.stride(0), _ptr(mem), mem.stride(0), _ptr(kcache), _ptr(vcache),
+                                      _ptr(step), n, int(H), float(scale), _ptr(out), out.stride(0), _stream()),
+          "kv_decode_attention")
+    return out
+
+
+def sample_tokens(logits, vocab, step, tokens, eos, temperature=None, seed=None, uniforms=None, forced=None, max_len=30,
+                  wte=None, wpe=None, emb_add=None, x_next=None):
+    """Draws tokens[:, t+1] from softmax(logits[:, :vocab] / temperature) (t = *step) and, with x_next, embeds it for the
+    next step.  logits fp32 [n, >=vocab]; temperature fp32 [1] and seed int64 [1] device tensors; uniforms fp32 [n, >=29]
+    replaces Philox; forced int32 [n, ldt] replaces sampling."""
+    _need(tokens, torch.int32, "tokens"); _need(step, torch.int32, "step"); _need(logits, torch.float32, "logits", True)
+    _need(temperature, torch.float32, "temperature"); _need(seed, torch.int64, "seed"); _need(uniforms, torch.float32, "uniforms")
+    _need(forced, torch.int32, "forced"); _need(wte, BF16, "wte"); _need(wpe, torch.float32, "wpe")
+    _need(emb_add, torch.float32, "emb_add", True); _need(x_next, BF16, "x_next", True)
+    n, ldt = tokens.shape
+    if forced is not None:
+        assert forced.shape == tokens.shape
+    C = wte.shape[1] if wte is not None else 0
+    check(lib.vdb_sample_tokens(_ptr(logits), logits.stride(0) if logits is not None else 0, int(vocab), n, _ptr(temperature),
+                                _ptr(step), _ptr(seed), _ptr(uniforms), uniforms.stride(0) if uniforms is not None else 0,
+                                _ptr(forced), int(eos), int(max_len), _ptr(tokens), ldt, _ptr(wte), _ptr(wpe), _ptr(emb_add),
+                                emb_add.stride(0) if emb_add is not None else 0, C, _ptr(x_next),
+                                x_next.stride(0) if x_next is not None else 0, _stream()), "sample_tokens")
+    return tokens
+
+
+def token_embed(tokens, wte, wpe, emb_add, out, step=None, pos_offset=1):
+    """out[r] = bf16(wte[tokens[r, t]] + wpe[t + pos_offset] + emb_add[r]), t = *step (0 without a counter)."""
+    _need(tokens, torch.int32, "tokens"); _need(wte, BF16, "wte"); _need(wpe, torch.float32, "wpe")
+    _need(emb_add, torch.float32, "emb_add", True); _need(out, BF16, "out", True); _need(step, torch.int32, "step")
+    n, ldt = tokens.shape
+    check(lib.vdb_token_embed(_ptr(tokens), ldt, _ptr(step), int(pos_offset), _ptr(wte), _ptr(wpe), _ptr(emb_add),
+                              emb_add.stride(0), n, wte.shape[1], _ptr(out), out.stride(0), _stream()), "token_embed")
     return out

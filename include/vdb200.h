@@ -25,7 +25,8 @@ extern "C" {
 
 enum { VDB_OK = 0, VDB_ERR_INVALID = 1, VDB_ERR_CUDA = 2, VDB_ERR_UNSUPPORTED = 3 };
 enum { VDB_ACT_NONE = 0, VDB_ACT_SILU = 1, VDB_ACT_GELU = 2, VDB_ACT_QUICK_GELU = 3, VDB_ACT_GEGLU = 4,
-       VDB_ACT_GELU_TANH = 5 /* GPT-2's tanh-form GELU, optimus_gpt2.py:99-100 */ };
+       VDB_ACT_GELU_TANH = 5 /* GPT-2's tanh-form GELU, optimus_gpt2.py:99-100 */,
+       VDB_ACT_TANH = 6 /* BertPooler's tanh, optimus_bert.py:364-376 */ };
 
 /* ---- library state ------------------------------------------------------------------------- */
 const char* vdb_version(void);
@@ -130,6 +131,16 @@ int vdb_attention_dv_pad(int d_head);
 int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, long long ldk, int k_col0,
                        const void* Vt, long long ldv, void* out, long long ldo, int B, int H, int Nq, int Nk,
                        int q_bstride, int kv_bstride, int d_head, float scale, int causal, void* stream);
+/* The same attention with a key count per batch item — BertSelfAttention with the padding mask of
+ * BertForLatentConnector_XX.forward (optimus_bert.py:1349-1439), whose keys are a prefix [CLS] .. [SEP] of every padded row.
+ * kv_len: device int [B]; batch item b attends to keys j < kv_len[b] only (values clamped to [1, Nk]).  The reference adds
+ * -10000 to the scores of the pad keys instead; with at least one real key in the row ([CLS] always is) exp(s - 10000 - max)
+ * is exactly 0 in fp32 for any score range a trained BERT produces, so leaving those keys out is the same softmax.  Runs the
+ * single-tile kernel only, d_head 49..64 (BERT's 64); with every kv_len[b] == Nk the result equals vdb_attention_bf16's bit for bit. */
+int vdb_attention_keylen_bf16(const void* Q, long long ldq, int q_col0, const void* K, long long ldk, int k_col0,
+                              const void* Vt, long long ldv, void* out, long long ldo, int B, int H, int Nq, int Nk,
+                              int q_bstride, int kv_bstride, int d_head, float scale, int causal, const int* kv_len,
+                              void* stream);
 
 /* ---- GroupNorm(32) [+SiLU] [+channel concat] on NHWC — normalization()/Normalize():
  *      diffusion_utils.py:168-191 (eps 1e-5), attention.py:76-77 & autokl_modules.py:38-39 (1e-6) ----
@@ -255,6 +266,15 @@ int vdb_sample_tokens(const float* logits, long long ldl, int V, int n, const fl
 /* x[row] = bf16(wte[tokens[row, t]] + wpe[t + pos_offset] + emb_add[row]), t = *step (0 when step == NULL): the <BOS> input. */
 int vdb_token_embed(const int* tokens, int ldt, const int* step, int pos_offset, const void* wte, const float* wpe,
                     const float* emb_add, long long ld_emb, int n, int C, void* x, long long ldx, void* stream);
+
+/* ---- Optimus BERT text encode — optimus_vae_next.encode (lib/model_zoo/optimus.py:729-743) on BertForLatentConnector_XX
+ *      (optimus_models/optimus_bert.py:1349-1439).  The 12 post-LN layers run on vdb_gemm_bf16 / vdb_attention_keylen_bf16 /
+ *      vdb_layernorm, the pooler on the VDB_ACT_TANH epilogue. ---------------------------------------------------------- */
+/* BertEmbeddings.forward (optimus_bert.py:144-175) with positions 0.. and token type 0: for ids int32 [n, L] (row-major),
+ * y[b*L + j] = bf16(LayerNorm(word_emb[ids[b, j]] + pos_emb[j] + type_emb[0]) * gamma + beta), fp32 throughout, the fp32
+ * tables read in place.  C % 128 == 0, C <= 1024, L <= max_pos; ids outside [0, vocab) are clamped. */
+int vdb_bert_embed_ln(const int* ids, int n, int L, const float* word_emb, int vocab, const float* pos_emb, int max_pos,
+                      const float* type_emb, const float* gamma, const float* beta, float eps, int C, void* y, void* stream);
 
 #ifdef __cplusplus
 }

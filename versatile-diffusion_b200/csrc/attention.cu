@@ -42,6 +42,7 @@ struct alignas(64) AttnParams {
   __nv_bfloat16* out;
   long long ldo;
   unsigned long long* timeline;   // debug (-DVDB_TIMELINE): per-tile role timestamps of CTA (0,0,0); null = off
+  const int* kv_len;              // per-batch key counts [B] of the KL = 1 kernels, clamped to [1, Nk]
 };
 
 // Debug build only (tools/attention_timeline.py): globaltimer stamps of one softmax warp (warp 2: lane quarter 2, first
@@ -75,7 +76,8 @@ constexpr int attention_ctas_per_sm() {   // by TMEM columns (512 per SM) and sh
   return (cols <= 128 && smem <= 75 * 1024) ? 3 : ((cols <= 256 && smem <= 113 * 1024) ? 2 : 1);
 }
 
-template <int DK, int DVP, int BKV, int KV_STAGES, int SB, int PB, int SW>
+// KL = 1: per-batch key counts p.kv_len (vdb_attention_keylen_bf16); KL = 0 compiles to the kernel without them.
+template <int DK, int DVP, int BKV, int KV_STAGES, int SB, int PB, int SW, int KL>
 __global__ void __launch_bounds__(64 + 128 * SW, attention_ctas_per_sm<DK, DVP, BKV, KV_STAGES, SB, PB>())
 attention_kernel(const __grid_constant__ AttnParams p) {
   constexpr int kBKV = BKV;
@@ -122,6 +124,7 @@ attention_kernel(const __grid_constant__ AttnParams p) {
   const int head = blockIdx.y;
   const int b = blockIdx.z;
 
+  int nk = 0;        // keys of this batch item (KL = 1; the KL = 0 kernels read p.Nk, a constant-bank operand)
   int ntiles = (p.Nk + kBKV - 1) / kBKV;
   if (p.causal) ntiles = min(ntiles, (q0 + kBQ + kBKV - 1) / kBKV);
 
@@ -148,6 +151,13 @@ attention_kernel(const __grid_constant__ AttnParams p) {
   const uint32_t tmem_base = *tmem_holder;
   pdl_launch_dependents();
   pdl_wait();
+  if constexpr (KL) {
+    // the batch item's own key count (read after the wait: an earlier kernel may have written it): the tiles past it are
+    // never loaded and the last tile masks the columns past it, exactly like the columns past Nk
+    nk = min(max(__ldg(p.kv_len + b), 1), p.Nk);
+    ntiles = (nk + kBKV - 1) / kBKV;
+    if (p.causal) ntiles = min(ntiles, (q0 + kBQ + kBKV - 1) / kBKV);
+  }
   const uint32_t tmem_S = tmem_base;             // SB x BKV columns
   const uint32_t tmem_O = tmem_base + SB * BKV;  // DVP columns
 
@@ -249,7 +259,8 @@ attention_kernel(const __grid_constant__ AttnParams p) {
       VDB_ATL(1, j, tl_warp);
       const uint32_t ts = tmem_S + (j % SB) * BKV + lane_off;
       const int kv0 = j * kBKV;
-      const int kv_lim = p.causal ? min(p.Nk, q_idx + 1) : p.Nk;  // valid kv indices are < kv_lim
+      const int nk_b = KL ? nk : p.Nk;
+      const int kv_lim = p.causal ? min(nk_b, q_idx + 1) : nk_b;  // valid kv indices are < kv_lim
       // pass 1: row max over this warp's columns.  With SW == 2 a thread owns only 64 columns, so the scores stay in
       // registers for pass 2 and S is read from TMEM once per tile instead of twice.
       float mx = -INFINITY;
@@ -411,7 +422,7 @@ attention_kernel(const __grid_constant__ AttnParams p) {
     };
 #pragma unroll 1
     for (int j = 0; j < ntiles; ++j) {
-      if ((j * kBKV + kBKV > p.Nk) || p.causal) tile_body(j, std::true_type{});
+      if ((j * kBKV + kBKV > (KL ? nk : p.Nk)) || p.causal) tile_body(j, std::true_type{});
       else tile_body(j, std::false_type{});
     }
     // epilogue: O / l -> bf16
@@ -884,11 +895,11 @@ struct AttnArgs {   // what the C ABI received; the tensor maps depend on the ke
   int B, H, q_bstride, kv_bstride;
 };
 
-template <int DK, int DVP, int BKV, int KV_STAGES, int SB, int PB, int SW>
+template <int DK, int DVP, int BKV, int KV_STAGES, int SB, int PB, int SW, int KL = 0>
 static int launch_attention(AttnParams& p, const AttnArgs& a, cudaStream_t stream) {
   constexpr size_t smem = attention_smem_bytes<DK, DVP, BKV>(KV_STAGES, PB);
   static_assert(smem <= 227 * 1024, "attention smem budget");
-  auto kernel = attention_kernel<DK, DVP, BKV, KV_STAGES, SB, PB, SW>;
+  auto kernel = attention_kernel<DK, DVP, BKV, KV_STAGES, SB, PB, SW, KL>;
   static bool configured = false;
   if (!configured) {
     VDB_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
@@ -981,9 +992,10 @@ int vdb_attention_dv_pad(int d_head) {
   return -1;
 }
 
-int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, long long ldk, int k_col0,
-                       const void* Vt, long long ldv, void* out, long long ldo, int B, int H, int Nq, int Nk,
-                       int q_bstride, int kv_bstride, int d_head, float scale, int causal, void* stream) {
+static int attention_entry(const void* Q, long long ldq, int q_col0, const void* K, long long ldk, int k_col0,
+                           const void* Vt, long long ldv, void* out, long long ldo, int B, int H, int Nq, int Nk,
+                           int q_bstride, int kv_bstride, int d_head, float scale, int causal, const int* kv_len,
+                           void* stream) {
   if (!Q || !K || !Vt || !out || B <= 0 || H <= 0 || Nq <= 0 || Nk <= 0)
     return set_error(VDB_ERR_INVALID, "attention: null/empty argument");
   const int DK = vdb_attention_dk_pad(d_head), DVP = vdb_attention_dv_pad(d_head);
@@ -1000,6 +1012,7 @@ int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, 
   memset(&p, 0, sizeof(p));
   const AttnArgs a{Q, K, Vt, ldq, ldk, ldv, B, H, q_bstride, kv_bstride};
   p.Nq = Nq; p.Nk = Nk; p.q_bs = q_bstride; p.kv_bs = kv_bstride; p.q_col0 = q_col0; p.k_col0 = k_col0; p.dv = d_head; p.causal = causal;
+  p.kv_len = kv_len;
   p.scale_log2 = scale * 1.4426950408889634f;
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
   p.ldo = ldo;
@@ -1017,7 +1030,8 @@ int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, 
   // pipe (0..4), T = 1 MUFU token / 0 free-running.  Without the ones row 11 was best (329 us on the B = 8, N = 4096, d = 40 launch;
   // 1 -> 358, 21 -> 334, 31 -> 334, 10 -> 340: profiles/r02_visit_f_summary.log).
   static const int fa = [] { const char* e = getenv("VDB_ATT_FA"); return e ? atoi(e) : -1; }();
-  if (fa != 0 && DK == 64 && !causal && Nk >= 512 && Nq >= 256 && (Nq % 256) == 0) {
+  // (per-batch key counts only exist in the kernel below: the two-tile kernel masks the last tile of Nk)
+  if (fa != 0 && !kv_len && DK == 64 && !causal && Nk >= 512 && Nq >= 256 && (Nq % 256) == 0) {
     // default: 3 of 8 pairs on the FMA pipe when the row sums come out of the tensor core (ONES: 315 us; 2 -> 318, 1 -> 340),
     // 1 of 8 otherwise (328 us; profiles/r02_visit_o_attention_ones.log)
     static const int ones_on = [] { const char* e = getenv("VDB_ATT_ONES"); return (e && e[0] == '0') ? 0 : 1; }();
@@ -1026,6 +1040,11 @@ int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, 
     if (DVP == 64) return dispatch_attention_fa<64>(mode, p, a, st);
   }
   static const int bkv = [] { const char* e = getenv("VDB_ATT_BKV"); const int v = e ? atoi(e) : 0; return (v == 64 || v == 643 || v == 128) ? v : 0; }();
+  if (kv_len) {   // the default tile choice below for BERT's d_head 64, with per-batch key counts
+    if (DK != 64 || DVP != 64) return set_error(VDB_ERR_UNSUPPORTED, "attention_keylen: d_head %d (needs 49..64)", d_head);
+    if (Nk > 64 && Nk <= 512) return launch_attention<64, 64, 64, 2, 1, 1, 2, 1>(p, a, st);
+    return launch_attention<64, 64, 128, 2, 1, 1, 2, 1>(p, a, st);
+  }
   if (sw == 2) {
     if (bkv == 64 && Nk > 64) {
       if (DK == 64 && DVP == 48) return launch_attention<64, 48, 64, 4, 2, 2, 2>(p, a, st);
@@ -1046,6 +1065,22 @@ int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, 
     if (DK == 192 && DVP == 160) return launch_attention<192, 160, 128, 1, 2, 2, 1>(p, a, st);
   }
   return set_error(VDB_ERR_UNSUPPORTED, "attention: no kernel for d_head %d", d_head);
+}
+
+int vdb_attention_bf16(const void* Q, long long ldq, int q_col0, const void* K, long long ldk, int k_col0,
+                       const void* Vt, long long ldv, void* out, long long ldo, int B, int H, int Nq, int Nk,
+                       int q_bstride, int kv_bstride, int d_head, float scale, int causal, void* stream) {
+  return attention_entry(Q, ldq, q_col0, K, ldk, k_col0, Vt, ldv, out, ldo, B, H, Nq, Nk, q_bstride, kv_bstride, d_head,
+                         scale, causal, nullptr, stream);
+}
+
+int vdb_attention_keylen_bf16(const void* Q, long long ldq, int q_col0, const void* K, long long ldk, int k_col0,
+                              const void* Vt, long long ldv, void* out, long long ldo, int B, int H, int Nq, int Nk,
+                              int q_bstride, int kv_bstride, int d_head, float scale, int causal, const int* kv_len,
+                              void* stream) {
+  if (!kv_len) return set_error(VDB_ERR_INVALID, "attention_keylen: kv_len is null");
+  return attention_entry(Q, ldq, q_col0, K, ldk, k_col0, Vt, ldv, out, ldo, B, H, Nq, Nk, q_bstride, kv_bstride, d_head,
+                         scale, causal, kv_len, stream);
 }
 
 }  // extern "C"

@@ -58,7 +58,7 @@ struct alignas(64) IgemmParams {
   void* out;                  // bf16 or fp32 [M, ldo]
   long long ldo;
   int out_f32;                // 1: fp32 output
-  int act;                    // 0 none, 1 silu, 2 gelu(erf), 3 quick_gelu, 4 geglu (packed halves), 5 gelu(tanh)
+  int act;                    // 0 none, 1 silu, 2 gelu(erf), 3 quick_gelu, 4 geglu (packed halves), 5 gelu(tanh), 6 tanh
   float alpha;                // out = act(alpha * (acc + bias)) + resid
   float* partial;             // split-K: [ksplit, M, N] fp32
   // LayerNorm folded into the GEMM (modes 5 / 6 consume, mode 7 produces; see the epilogue):
@@ -78,7 +78,7 @@ struct alignas(64) IgemmParams {
   int chunked;                // 1: every CTA walks a contiguous range of tiles instead of a grid-strided one
 };
 
-enum { ACT_NONE = 0, ACT_SILU = 1, ACT_GELU = 2, ACT_QGELU = 3, ACT_GEGLU = 4, ACT_GELU_TANH = 5 };
+enum { ACT_NONE = 0, ACT_SILU = 1, ACT_GELU = 2, ACT_QGELU = 3, ACT_GEGLU = 4, ACT_GELU_TANH = 5, ACT_TANH = 6 };
 
 #ifdef VDB_TIMELINE   // debug build only (tools/gemm_timeline.py): per-tile role timestamps of CTA 0
 #define VDB_TL(slot, it) do { if (p.timeline && blockIdx.x == 0 && (it) < 8) p.timeline[(it) * 16 + (slot)] = gtime(); } while (0)
@@ -109,6 +109,7 @@ VDB_DEVINL float apply_act(float v, int act) {
     case ACT_GELU: return gelu_erf_f(v);
     case ACT_QGELU: return quick_gelu_f(v);
     case ACT_GELU_TANH: return gelu_tanh_f(v);
+    case ACT_TANH: return tanhf(v);
     default: return v;
   }
 }

@@ -4,7 +4,8 @@ The reference resolves YAML with `super_cfg` inheritance and MODEL(name) indirec
 are the resolved results for the shipped configs (configs/model/{vd,openai_unet,autokl,clip}.yaml).
 By default 'vd_four_flow_v1-0' carries the image VAE, both CLIP context encoders, the 2D diffuser and the 0D diffuser's
 context blocks.  VDB_TEXT_FLOWS=1 adds what the text-latent flows (i2t / t2t) need: the 0D diffuser's data blocks and the
-Optimus text VAE's decoder (configs/model/optimus.yaml), registered as vae['text'].
+Optimus text VAE's decoder (configs/model/optimus.yaml), registered as vae['text']; VDB_TEXT_ENCODER=1 on top of it adds the
+text VAE's BERT encoder (vae_encode(x, 'text')).
 """
 import copy
 import os
@@ -78,9 +79,16 @@ _BANK = {
     "vd_base": dict(symbol="vd", find_unused_parameters=True, type="vd_v2_0", args=dict(
         beta_linear_start=0.00085, beta_linear_end=0.012, timesteps=1000, use_ema=False)),
 }
-# configs/model/optimus.yaml:43-90, 96-102 with MODEL(...) resolved; only the decoder side is built (the BERT encoder is used
-# by no app.py flow), and the training-only fields (dropouts, summary heads) are left out
+# configs/model/optimus.yaml:7-41, 43-90, 96-102 with MODEL(...) resolved, without the training-only fields (dropouts, summary
+# heads, the MLM head's settings); optimus_v1 carries the BERT encoder only with VDB_TEXT_ENCODER=1 (no app.py flow encodes text)
 _TEXT_BANK = {
+    "optimus_bert_encoder": dict(symbol="optimus", find_unused_parameters=False, type="optimus_bert_connector", args=dict(
+        config=dict(hidden_act="gelu", hidden_size=768, initializer_range=0.02, intermediate_size=3072, layer_norm_eps=1e-12,
+                    max_position_embeddings=512, num_attention_heads=12, num_hidden_layers=12, type_vocab_size=2,
+                    vocab_size=28996),
+        latent_size=768)),
+    "optimus_bert_tokenizer": dict(symbol="optimus", find_unused_parameters=False, type="optimus_bert_tokenizer", args=dict(
+        do_lower_case=False, max_len=512, vocab_file="lib/model_zoo/optimus_models/vocab/bert-base-cased-vocab.txt")),
     "optimus_gpt2_decoder": dict(symbol="optimus", find_unused_parameters=False, type="optimus_gpt2_connector", args=dict(
         config=dict(hidden_size=768, initializer_range=0.02, latent_size=768, layer_norm_epsilon=1e-05,
                     max_position_embeddings=1024, n_ctx=1024, n_embd=768, n_head=12, n_layer=12, n_positions=1024,
@@ -96,6 +104,12 @@ _TEXT_BANK["optimus_v1"] = dict(symbol="optimus", find_unused_parameters=False, 
 
 def _text_flows():
     return os.environ.get("VDB_TEXT_FLOWS") == "1"
+
+
+def _text_encoder():
+    """VDB_TEXT_ENCODER=1 (together with VDB_TEXT_FLOWS=1): vae['text'] also builds the BERT encoder behind
+    vae_encode(x, 'text') / ctx_encode(x, 'vae_text') (+108 M parameters the i2t / t2t flows do not use)"""
+    return os.environ.get("VDB_TEXT_ENCODER") == "1"
 
 
 for _sfx, _parts in _PARTS.items():
@@ -118,7 +132,10 @@ class model_cfg_bank(object):
                 global_layer_ptr="image", latent_scale_factor={"image": 0.18215}))
             return cfg
         if _text_flows() and name in _TEXT_BANK:
-            return CfgDict(copy.deepcopy(_TEXT_BANK[name]))
+            cfg = CfgDict(copy.deepcopy(_TEXT_BANK[name]))
+            if name == "optimus_v1" and _text_encoder():
+                cfg.args.update(dict(encoder=self("optimus_bert_encoder"), tokenizer_encoder=self("optimus_bert_tokenizer")))
+            return cfg
         if name not in _BANK:
             raise KeyError(f"config '{name}' is outside the B200 hot-path build (have: {sorted(_BANK)} + vd_four_flow_v1-0; "
                            "VDB_TEXT_FLOWS=1 adds the Optimus text VAE)")

@@ -1,5 +1,5 @@
-"""Optimus text VAE (decoder side) on vdb200 kernels — reference lib/model_zoo/optimus.py:17-52, 645-763 and
-optimus_models/optimus_gpt2.py:99-246, 813-1112.
+"""Optimus text VAE on vdb200 kernels — reference lib/model_zoo/optimus.py:17-52, 636-763,
+optimus_models/optimus_gpt2.py:99-246, 813-1112 (decoder) and optimus_models/optimus_bert.py:144-376, 1349-1439 (encoder).
 
 `optimus_vae_next.decode(z)` turns text latents [n, 768] into sentences like the reference's: a GPT-2 decoder that sees the
 latent twice — `linear_emb(z)` added to every input embedding and one slice of `linear(z)` per layer used as a one-slot past
@@ -7,11 +7,17 @@ key AND value — samples up to 30 tokens from `<BOS>`.  The reference re-runs t
 the host; here every layer keeps a bf16 KV cache, the sampler runs on the device, and the token step is one captured CUDA
 graph replayed 28 times, so the host sees only the final [n, 30] token ids.
 
-The module tree keeps the reference's state_dict keys and shapes (`decoder.transformer.*`, `decoder.lm_head` tied to
-`wte`); only the decoder is built.  The BERT encoder (`vae_encode(., 'text')`) is used by no app.py flow.
+`optimus_vae_next.encode(sentences)` maps sentences to the latent mean z_mu [n, 768] like the reference: a clean-room BERT
+WordPiece tokenizer on the host, one copy of the padded ids to the device, then a post-LN BERT-base encoder whose attention
+leaves every sentence's pad keys out (vdb_attention_keylen_bf16), the tanh pooler on [CLS] and the first half of `linear`.
+
+The module trees keep the reference's state_dict keys and shapes (`decoder.transformer.*`, `decoder.lm_head` tied to `wte`;
+`encoder.embeddings.*`, `encoder.encoder.layer.N.*`, `encoder.pooler.dense`, `encoder.linear`).  The encoder is built only
+when the VAE is given one (VDB_TEXT_ENCODER=1 in lib/cfg_helper.py): no app.py flow encodes text.
 """
 import json
 import os
+import unicodedata
 
 import torch
 import torch.nn as nn
@@ -26,6 +32,9 @@ MAX_LENGTH = 30                                        # optimus.py:751
 CACHE_SLOTS = 32                                       # KV-cache slots per (row, head), vdb_kv_decode_attention
 D_HEAD = 64
 DEFAULT_VOCAB = "lib/model_zoo/optimus_models/vocab/gpt2-vocab.json"
+DEFAULT_BERT_VOCAB = "lib/model_zoo/optimus_models/vocab/bert-base-cased-vocab.txt"
+BERT_PAD_ID = 0                                        # pad_sequence's padding_value (optimus.py:739); [PAD] in the vocabulary
+BERT_MAX_PIECES = 510                                  # + [CLS] + [SEP] = the 512 rows of the position table
 
 
 def _ops():
@@ -318,11 +327,270 @@ def truncate_at_eos(row):
     return row[:row.index(EOS_ID) + 1] if EOS_ID in row else row
 
 
+# ------------------------------------------------------------------------------------------------ BERT encoder
+class _Linear(nn.Linear):
+    def __init__(self, n_in, n_out, bias=True, std=0.02):
+        super().__init__(n_in, n_out, bias=bias)
+        self.weight.data.normal_(std=std)                  # _init_weights of the reference (optimus_bert.py:1371-1381)
+        if bias:
+            self.bias.data.zero_()
+
+
+class BertEmbeddings(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        self.word_embeddings = nn.Embedding(c["vocab_size"], c["hidden_size"], padding_idx=0)
+        self.position_embeddings = nn.Embedding(c["max_position_embeddings"], c["hidden_size"])
+        self.token_type_embeddings = nn.Embedding(c["type_vocab_size"], c["hidden_size"])
+        self.LayerNorm = nn.LayerNorm(c["hidden_size"], eps=c["layer_norm_eps"])
+        for e in (self.word_embeddings, self.position_embeddings, self.token_type_embeddings):
+            e.weight.data.normal_(std=c.get("initializer_range", 0.02))
+
+
+class BertSelfAttention(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        C, std = c["hidden_size"], c.get("initializer_range", 0.02)
+        self.query, self.key, self.value = _Linear(C, C, std=std), _Linear(C, C, std=std), _Linear(C, C, std=std)
+
+
+class BertSelfOutput(nn.Module):
+    def __init__(self, c, n_in):
+        super().__init__()
+        self.dense = _Linear(n_in, c["hidden_size"], std=c.get("initializer_range", 0.02))
+        self.LayerNorm = nn.LayerNorm(c["hidden_size"], eps=c["layer_norm_eps"])
+
+
+class BertAttention(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        self.self = BertSelfAttention(c)
+        self.output = BertSelfOutput(c, c["hidden_size"])
+
+
+class BertIntermediate(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        self.dense = _Linear(c["hidden_size"], c["intermediate_size"], std=c.get("initializer_range", 0.02))
+
+
+class BertLayer(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        self.attention = BertAttention(c)
+        self.intermediate = BertIntermediate(c)
+        self.output = BertSelfOutput(c, c["intermediate_size"])     # BertOutput: dense + LayerNorm, the same tree
+
+
+class BertEncoder(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        self.layer = nn.ModuleList([BertLayer(c) for _ in range(c["num_hidden_layers"])])
+
+
+class BertPooler(nn.Module):
+    def __init__(self, c):
+        super().__init__()
+        self.dense = _Linear(c["hidden_size"], c["hidden_size"], std=c.get("initializer_range", 0.02))
+
+
+@register('optimus_bert_connector')
+class BertForLatentConnector_XX(PackedMixin, nn.Module):
+    """optimus_bert.py:1349-1439 as optimus_vae_next.encode uses it: post-LN BERT (exact-erf GELU), the tanh pooler on [CLS],
+    and `linear` (hidden -> 2 * latent, no bias) whose first half is the latent mean."""
+
+    def __init__(self, config, latent_size=32):
+        super().__init__()
+        self.config = dict(config)
+        c = self.config
+        if c.get("hidden_act", "gelu") != "gelu":
+            raise NotImplementedError(f"hidden_act {c['hidden_act']!r}: only BERT's exact-erf 'gelu' is built")
+        self.latent_size = latent_size
+        self.embeddings = BertEmbeddings(c)
+        self.encoder = BertEncoder(c)
+        self.pooler = BertPooler(c)
+        self.linear = _Linear(c["hidden_size"], 2 * latent_size, bias=False, std=c.get("initializer_range", 0.02))
+
+    def _pack(self):
+        c = self.config
+        C, H = c["hidden_size"], c["num_attention_heads"]
+        if C != H * D_HEAD or C % 128:
+            raise NotImplementedError(f"the encode kernels need d_head = {D_HEAD} and a width that is a multiple of 128 "
+                                      f"(hidden_size {C}, {H} heads)")
+        e = self.embeddings
+        layers = []
+        for ly in self.encoder.layer:
+            a = ly.attention
+            wo = a.output.dense.weight.detach().float()
+            layers.append(dict(
+                wqk=bf16(torch.cat([a.self.query.weight.detach(), a.self.key.weight.detach()], 0)),
+                bqk=f32(torch.cat([a.self.query.bias.detach(), a.self.key.bias.detach()], 0)),
+                wv=bf16(a.self.value.weight),
+                # softmax rows sum to 1 over the kept keys too, so P(V + 1 b_v^T) = PV + b_v: the V bias moves through the output
+                wo=bf16(wo), bo=(a.output.dense.bias.detach().float() + wo @ a.self.value.bias.detach().float()).contiguous(),
+                ln1=(f32(a.output.LayerNorm.weight), f32(a.output.LayerNorm.bias)),
+                w1=bf16(ly.intermediate.dense.weight), b1=f32(ly.intermediate.dense.bias),
+                w2=bf16(ly.output.dense.weight), b2=f32(ly.output.dense.bias),
+                ln2=(f32(ly.output.LayerNorm.weight), f32(ly.output.LayerNorm.bias))))
+        return dict(layers=layers, word=f32(e.word_embeddings.weight), pos=f32(e.position_embeddings.weight),
+                    type0=f32(e.token_type_embeddings.weight[0]), emb_ln=(f32(e.LayerNorm.weight), f32(e.LayerNorm.bias)),
+                    eps=float(c["layer_norm_eps"]), pool_w=bf16(self.pooler.dense.weight), pool_b=f32(self.pooler.dense.bias),
+                    mu_w=bf16(self.linear.weight[:self.latent_size]), heads=H, width=C)
+
+    @torch.no_grad()
+    def encode_ids(self, ids, lengths, n_keys):
+        """ids int32 [n, Lp] on the device (rows padded with 0 to Lp, a multiple of 8), lengths int32 [n] on the device (the
+        ids of row b before its padding, [CLS] .. [SEP]), n_keys = max(lengths) on the host -> fp32 z_mu [n, latent].
+        About 8 launches per layer plus 3."""
+        require_cuda(ids, "optimus encode")
+        ops, pk = _ops(), self.packed()
+        n, Lp = ids.shape
+        C, H, eps = pk["width"], pk["heads"], pk["eps"]
+        if Lp % 8 or not 1 <= n_keys <= Lp:
+            raise ValueError(f"encode_ids: padded length {Lp} must be a multiple of 8 and hold the {n_keys} keys")
+        x = ops.bert_embed_ln(ids, pk["word"], pk["pos"], pk["type0"], *pk["emb_ln"], eps=eps)     # [n*Lp, C]
+        o = torch.zeros(n * Lp, C, dtype=torch.bfloat16, device=ids.device)      # rows past n_keys are never written
+        for ly in pk["layers"]:
+            qk = ops.gemm(x, ly["wqk"], bias=ly["bqk"])                           # [n*Lp, 2C]: q | k
+            vt = ops.gemm(ly["wv"], x)                                            # [C, n*Lp] = V^T (bias folded into bo)
+            ops.attention(qk, qk, vt, o, n, H, n_keys, n_keys, D_HEAD, scale=D_HEAD ** -0.5, q_col0=0, k_col0=C,
+                          q_bstride=Lp, kv_bstride=Lp, kv_len=lengths)
+            h = ops.layernorm(ops.gemm(o, ly["wo"], bias=ly["bo"], resid=x), *ly["ln1"], eps=eps)
+            f = ops.gemm(h, ly["w1"], bias=ly["b1"], act=ops.ACT_GELU)
+            x = ops.layernorm(ops.gemm(f, ly["w2"], bias=ly["b2"], resid=h), *ly["ln2"], eps=eps)
+        cls = x.view(n, Lp * C)[:, :C]                                            # the [CLS] rows: lda = Lp * C
+        pooled = ops.gemm(cls, pk["pool_w"], bias=pk["pool_b"], act=ops.ACT_TANH)
+        return ops.gemm(pooled, pk["mu_w"], out_dtype=torch.float32)
+
+
+def _is_bert_whitespace(ch):
+    return ch in " \t\n\r" or unicodedata.category(ch) == "Zs"
+
+
+def _is_bert_control(ch):
+    return ch not in "\t\n\r" and unicodedata.category(ch).startswith("C")
+
+
+def _is_bert_punctuation(ch):
+    cp = ord(ch)
+    return 33 <= cp <= 47 or 58 <= cp <= 64 or 91 <= cp <= 96 or 123 <= cp <= 126 or unicodedata.category(ch).startswith("P")
+
+
+_CJK_RANGES = ((0x4E00, 0x9FFF), (0x3400, 0x4DBF), (0x20000, 0x2A6DF), (0x2A700, 0x2B73F), (0x2B740, 0x2B81F),
+               (0x2B820, 0x2CEAF), (0xF900, 0xFAFF), (0x2F800, 0x2FA1F))
+
+
+def _is_cjk(ch):
+    cp = ord(ch)
+    return any(lo <= cp <= hi for lo, hi in _CJK_RANGES)
+
+
+@register('optimus_bert_tokenizer')
+class BertTokenizer(object):
+    """What optimus_vae_next.encode uses of the reference's BertTokenizer (tokenization_bert.py, tokenization_utils.py:576-625)
+    with do_lower_case = False: text cleaning (NUL, U+FFFD and control characters dropped, whitespace -> ' '), CJK characters
+    split out, whitespace and punctuation splits, accents kept, then greedy longest-match-first WordPiece ('##' continuations,
+    [UNK] for a word that cannot be covered or is longer than 100 characters).  Needs only the vocabulary file (one piece per
+    line, the line number is the id); VDB_BERT_VOCAB overrides its path.
+
+    A text that is all whitespace (but not empty) comes out of the reference as ONE special token picked by Python's set order
+    of the special-token strings, which changes with the hash seed of the process; here it is always [UNK]."""
+    max_input_chars_per_word = 100
+
+    def __init__(self, vocab_file=DEFAULT_BERT_VOCAB, do_lower_case=False, **kwargs):
+        if do_lower_case:
+            raise NotImplementedError("only the cased tokenizer of the Optimus encoder (do_lower_case = False) is built")
+        self.vocab_file = vocab_file
+        self._vocab_map = None
+
+    def vocab(self):
+        if self._vocab_map is None:
+            path = os.environ.get("VDB_BERT_VOCAB") or self.vocab_file
+            if not os.path.exists(path):
+                raise RuntimeError(f"BERT vocabulary '{path}' is not available (cwd {os.getcwd()}): run from the tree that holds "
+                                   f"{DEFAULT_BERT_VOCAB} or point VDB_BERT_VOCAB at a bert-base-cased-vocab.txt")
+            with open(path, encoding="utf-8") as fh:
+                self._vocab_map = {line.rstrip("\n"): i for i, line in enumerate(fh)}
+        return self._vocab_map
+
+    def _id(self, piece):
+        v = self.vocab()
+        return v.get(piece, v["[UNK]"])
+
+    @property
+    def cls_token_id(self):
+        return self._id("[CLS]")
+
+    @property
+    def sep_token_id(self):
+        return self._id("[SEP]")
+
+    @staticmethod
+    def basic_tokenize(text):
+        out = []
+        for ch in text:
+            if ch == "\x00" or ch == "\ufffd" or _is_bert_control(ch):
+                continue
+            if _is_bert_whitespace(ch):
+                out.append(" ")
+            elif _is_cjk(ch):
+                out.append(" " + ch + " ")
+            else:
+                out.append(ch)
+        words = []
+        for word in "".join(out).split():
+            cur = ""
+            for ch in word:
+                if _is_bert_punctuation(ch):
+                    if cur:
+                        words.append(cur)
+                        cur = ""
+                    words.append(ch)
+                else:
+                    cur += ch
+            if cur:
+                words.append(cur)
+        return words
+
+    def wordpiece(self, word):
+        if len(word) > self.max_input_chars_per_word:
+            return ["[UNK]"]
+        vocab = self.vocab()
+        pieces, start = [], 0
+        while start < len(word):
+            for end in range(len(word), start, -1):
+                piece = word[start:end] if start == 0 else "##" + word[start:end]
+                if piece in vocab:
+                    break
+            else:
+                return ["[UNK]"]
+            pieces.append(piece)
+            start = end
+        return pieces
+
+    def tokenize(self, text):
+        if text and not text.strip():
+            return ["[UNK]"]
+        return [p for w in self.basic_tokenize(text) for p in self.wordpiece(w)]
+
+    def convert_tokens_to_ids(self, pieces):
+        return [self._id(p) for p in pieces]
+
+    def encode_sentences(self, sentences, max_length=77):
+        """optimus.py:729-738: lower-case, tokenize, keep the first max_length pieces, add [CLS] .. [SEP] -> list of id lists"""
+        cls, sep = self.cls_token_id, self.sep_token_id
+        return [[cls] + self.convert_tokens_to_ids(self.tokenize(s.lower())[:max_length]) + [sep] for s in sentences]
+
+
 # ------------------------------------------------------------------------------------------------ the VAE surface
 @register('optimus_vae_next')
 class optimus_vae_next(nn.Module):
     def __init__(self, encoder=None, decoder=None, tokenizer_encoder=None, tokenizer_decoder=None, args=None):
         super().__init__()
+        if encoder is not None:
+            self.encoder = encoder if isinstance(encoder, nn.Module) else get_model()(encoder, verbose=False)
+            self.tokenizer_encoder = tokenizer_encoder if isinstance(tokenizer_encoder, BertTokenizer) \
+                else get_model()(tokenizer_encoder, verbose=False)
         self.decoder = decoder if isinstance(decoder, nn.Module) else get_model()(decoder, verbose=False)
         self.tokenizer_decoder = tokenizer_decoder if isinstance(tokenizer_decoder, GPT2Detokenizer) \
             else get_model()(tokenizer_decoder, verbose=False)
@@ -333,9 +601,29 @@ class optimus_vae_next(nn.Module):
     def get_device(self):
         return self.decoder.transformer.linear.weight.device
 
+    @torch.no_grad()
     def encode(self, text, max_length=77):
-        raise NotImplementedError("Optimus text encoding (the BERT encoder, vae_encode(x, 'text')) is not built: no app.py flow "
-                                  "uses it; only decode() is available")
+        """optimus.py:729-743: sentences (a list of str; a single str is one sentence) -> fp32 z_mu [n, latent] on the device.
+        Each sentence keeps its first max_length word pieces; the rows are padded to the longest, rounded up to 8."""
+        if getattr(self, "encoder", None) is None:
+            raise NotImplementedError("Optimus text encoding (the BERT encoder, vae_encode(x, 'text')) is not built in this VAE: "
+                                      "construct it with an encoder (VDB_TEXT_FLOWS=1 VDB_TEXT_ENCODER=1 in the config bank)")
+        if not 0 <= max_length <= BERT_MAX_PIECES:
+            raise ValueError(f"max_length {max_length}: at most {BERT_MAX_PIECES} pieces fit the 512 positions with [CLS] and [SEP]")
+        sentences = [text] if isinstance(text, str) else list(text)
+        if not sentences:
+            raise ValueError("encode: no sentences")
+        rows = self.tokenizer_encoder.encode_sentences(sentences, max_length)
+        n, keys = len(rows), max(len(r) for r in rows)
+        Lp = (keys + 7) // 8 * 8                         # the attention's per-item row stride must stay 16-byte aligned
+        host = torch.full((n * Lp + n,), BERT_PAD_ID, dtype=torch.int32)
+        for b, r in enumerate(rows):
+            host[b * Lp:b * Lp + len(r)] = torch.tensor(r, dtype=torch.int32)
+            host[n * Lp + b] = len(r)
+        dev = self.encoder.linear.weight.device
+        require_cuda(self.encoder.linear.weight, "optimus encode")
+        buf = host.to(dev)                               # ids and lengths in one host-to-device copy
+        return self.encoder.encode_ids(buf[:n * Lp].view(n, Lp), buf[n * Lp:], keys)
 
     @torch.no_grad()
     def decode_tokens(self, z, temperature=1.0, uniforms=None, pre_scale=1.0, use_graph=True):

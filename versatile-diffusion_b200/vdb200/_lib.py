@@ -66,6 +66,8 @@ SIGNATURES = {
     "vdb_kv_decode_attention": (i, [p, ll, p, ll, p, p, p, i, i, f, p, ll, p]),
     "vdb_sample_tokens": (i, [p, ll, i, i, p, p, p, p, i, p, i, i, p, i, p, p, p, ll, i, p, ll, p]),
     "vdb_token_embed": (i, [p, i, p, i, p, p, p, ll, i, i, p, ll, p]),
+    "vdb_attention_keylen_bf16": (i, [p, ll, i, p, ll, i, p, ll, p, ll, i, i, i, i, i, i, i, f, i, p, p]),
+    "vdb_bert_embed_ln": (i, [p, i, i, p, i, p, i, p, p, p, f, i, p, p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -12,7 +12,7 @@ import torch
 
 from ._lib import lib, check
 
-ACT_NONE, ACT_SILU, ACT_GELU, ACT_QUICK_GELU, ACT_GEGLU, ACT_GELU_TANH = 0, 1, 2, 3, 4, 5
+ACT_NONE, ACT_SILU, ACT_GELU, ACT_QUICK_GELU, ACT_GEGLU, ACT_GELU_TANH, ACT_TANH = 0, 1, 2, 3, 4, 5, 6
 BF16 = torch.bfloat16
 
 
@@ -345,17 +345,23 @@ def attention_pads(d_head):
 
 
 def attention(q, k, vt, out, B, H, Nq, Nk, d_head, scale=None, q_col0=0, k_col0=0, causal=False,
-              q_bstride=0, kv_bstride=0):
+              q_bstride=0, kv_bstride=0, kv_len=None):
     """Flash attention. q [B*q_bstride, ldq], k [B*kv_bstride, ldk], vt [H*DVP, B*kv_bstride], out [B*q_bstride, H*d_head].
-    kv_bstride (default Nk) must be a multiple of 8: pad ragged contexts per batch item."""
+    kv_bstride (default Nk) must be a multiple of 8: pad ragged contexts per batch item.
+    kv_len: int32 device tensor [B] -> batch item b attends to its first kv_len[b] keys only (vdb_attention_keylen_bf16)."""
     _need(q, BF16, "q", True); _need(k, BF16, "k", True); _need(vt, BF16, "vt", True); _need(out, BF16, "out", True)
+    _need(kv_len, torch.int32, "kv_len")
+    if kv_len is not None and kv_len.numel() < B:
+        raise ValueError(f"kv_len: need one key count per batch item ({B}), got {kv_len.numel()}")
     if scale is None:
         scale = d_head ** -0.5
+    args = (_ptr(q), q.stride(0), int(q_col0), _ptr(k), k.stride(0), int(k_col0), _ptr(vt), vt.stride(0), _ptr(out),
+            out.stride(0), B, H, Nq, Nk, int(q_bstride), int(kv_bstride), d_head, float(scale), 1 if causal else 0)
     with _Span("attention", 4.0 * B * H * Nq * Nk * d_head, 2.0 * B * H * d_head * (2 * Nq + 2 * Nk)):
-        check(lib.vdb_attention_bf16(_ptr(q), q.stride(0), int(q_col0), _ptr(k), k.stride(0), int(k_col0), _ptr(vt),
-                                     vt.stride(0), _ptr(out), out.stride(0), B, H, Nq, Nk, int(q_bstride),
-                                     int(kv_bstride), d_head, float(scale), 1 if causal else 0, _stream()),
-              "attention_bf16")
+        if kv_len is None:
+            check(lib.vdb_attention_bf16(*args, _stream()), "attention_bf16")
+        else:
+            check(lib.vdb_attention_keylen_bf16(*args, _ptr(kv_len), _stream()), "attention_keylen_bf16")
     return out
 
 
@@ -689,4 +695,25 @@ def token_embed(tokens, wte, wpe, emb_add, out, step=None, pos_offset=1):
     n, ldt = tokens.shape
     check(lib.vdb_token_embed(_ptr(tokens), ldt, _ptr(step), int(pos_offset), _ptr(wte), _ptr(wpe), _ptr(emb_add),
                               emb_add.stride(0), n, wte.shape[1], _ptr(out), out.stride(0), _stream()), "token_embed")
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
+# Optimus BERT text encode (optimus.py:729-743): the embedding layer; the encoder layers use gemm / attention(kv_len) / layernorm
+# ------------------------------------------------------------------------------------------------
+def bert_embed_ln(ids, word_emb, pos_emb, type_emb, gamma, beta, eps=1e-12, out=None):
+    """ids int32 [n, L] -> bf16 [n*L, C] = LayerNorm(word_emb[ids] + pos_emb[:L] + type_emb[0]) (fp32 tables read in place)."""
+    _need(ids, torch.int32, "ids"); _need(word_emb, torch.float32, "word_emb"); _need(pos_emb, torch.float32, "pos_emb")
+    _need(type_emb, torch.float32, "type_emb"); _need(gamma, torch.float32, "gamma"); _need(beta, torch.float32, "beta")
+    n, L = ids.shape
+    C = word_emb.shape[1]
+    if pos_emb.shape[1] != C or type_emb.shape[-1] != C or gamma.numel() != C or beta.numel() != C:
+        raise ValueError(f"bert_embed_ln: tables of width {C}, {pos_emb.shape[1]}, {type_emb.shape[-1]}, gamma {gamma.numel()}, "
+                         f"beta {beta.numel()} disagree")
+    if out is None:
+        out = torch.empty((n * L, C), dtype=BF16, device=ids.device)
+    _need(out, BF16, "out")
+    assert out.shape == (n * L, C), (tuple(out.shape), n * L, C)
+    check(lib.vdb_bert_embed_ln(_ptr(ids), n, L, _ptr(word_emb), word_emb.shape[0], _ptr(pos_emb), pos_emb.shape[0],
+                                _ptr(type_emb), _ptr(gamma), _ptr(beta), float(eps), C, _ptr(out), _stream()), "bert_embed_ln")
     return out

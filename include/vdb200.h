@@ -121,7 +121,8 @@ int vdb_conv3x3_bf16(const void* X, int B, int H, int W, int C, int mode, const 
  * O = softmax(Q K^T * scale) V per (batch, head), fp32 online softmax, nothing materialised.
  * Q [B*Nq, ldq] head h at columns q_col0 + h*DK; K [B*Nk, ldk] at k_col0 + h*DK;
  * Vt [H*DVP, ldv] row h*DVP + c, column b*Nk + j; out [B*Nq, ldo] head h at columns h*d_head.
- * DK = vdb_attention_dk_pad(d_head), DVP = vdb_attention_dv_pad(d_head); pad columns/rows must be
+ * DK = vdb_attention_dk_pad(d_head), DVP = vdb_attention_dv_pad(d_head): (64, 48) up to d_head 48, (64, 64) up to 64,
+ * (128, 80) up to 80, (192, 160) up to 160 (d_head a multiple of 8); pad columns/rows must be
  * zero (the projection weights are zero-padded at pack time). causal != 0: CLIP text mask.
  * Batch b starts at row b*q_bstride of Q/out and at row (K) / column (Vt) b*kv_bstride; kv_bstride must be a
  * multiple of 8 (TMA: 16-byte aligned innermost coordinate), so ragged contexts (77, 257 tokens) are stored

@@ -32,6 +32,10 @@ def test_host_side_argument_checks_without_gpu():
     assert lib.vdb_gemm_bf16(None, 0, 0, 0, None, 0, 0, None, 0, 0, None, 0, 0, None, 0, None, 0, 0, 0, 1.0, 0, 0, None, 0, None) == 1
     assert lib.vdb_attention_dk_pad(40) == 64 and lib.vdb_attention_dv_pad(40) == 48
     assert lib.vdb_attention_dk_pad(160) == 192 and lib.vdb_attention_dv_pad(160) == 160
+    # one (DK, DVP) pair per attention kernel: d_head 81..160 share the (192, 160) one
+    assert [lib.vdb_attention_dk_pad(d) for d in (8, 64, 72, 80, 88, 96, 120, 128, 136)] == [64, 64, 128, 128, 192, 192, 192, 192, 192]
+    assert [lib.vdb_attention_dv_pad(d) for d in (48, 56, 80, 88, 128)] == [48, 64, 80, 160, 160]
+    assert lib.vdb_attention_dk_pad(168) == -1 and lib.vdb_attention_dv_pad(168) == -1
     assert lib.vdb_attention_dk_pad(512) == -1
 
 

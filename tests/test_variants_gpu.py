@@ -1,6 +1,6 @@
 """Opt-in kernel variants (environment switches read once per process) against the same kernel parity tests, each in its own
 process.  Skipped unless VDB_TEST_VARIANTS=1: variants that have not been measured/validated on a B200 yet stay out of the
-default GPU suite (the default kernels are covered by test_kernels_gpu.py / test_parity_gpu.py)."""
+default GPU suite (the default kernels are covered by test_kernels_gpu.py / test_kernel_edges_gpu.py / test_parity_gpu.py)."""
 import os
 import subprocess
 import sys
@@ -35,7 +35,8 @@ RUN = pytest.mark.skipif(os.environ.get("VDB_TEST_VARIANTS") != "1", reason="set
 def test_variant(env, select):
     e = dict(os.environ, **env)
     out = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "--timeout", "120",
-                          os.path.join(ROOT, "tests", "test_kernels_gpu.py"), "-k", select],
+                          os.path.join(ROOT, "tests", "test_kernels_gpu.py"), os.path.join(ROOT, "tests", "test_kernel_edges_gpu.py"),
+                          "-k", select],
                          capture_output=True, text=True, env=e, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-1000:]
 

@@ -895,6 +895,11 @@ struct AttnArgs {   // what the C ABI received; the tensor maps depend on the ke
   int B, H, q_bstride, kv_bstride;
 };
 
+// debug aid: which kernel family the last attention call on this thread launched (vdb_debug_attention_last)
+enum { kAttNone = 0, kAttTwoTile = 1, kAttCols64Dbuf = 2, kAttCols64ThreeCta = 3, kAttCols128 = 4, kAttD80 = 5, kAttD160 = 6,
+       kAttKeylen64 = 7, kAttKeylen128 = 8 };
+static thread_local int g_att_last = kAttNone;
+
 template <int DK, int DVP, int BKV, int KV_STAGES, int SB, int PB, int SW, int KL = 0>
 static int launch_attention(AttnParams& p, const AttnArgs& a, cudaStream_t stream) {
   constexpr size_t smem = attention_smem_bytes<DK, DVP, BKV>(KV_STAGES, PB);
@@ -913,6 +918,8 @@ static int launch_attention(AttnParams& p, const AttnArgs& a, cudaStream_t strea
   rc = make_tmap_2d(&p.tmV, a.Vt, static_cast<uint64_t>(a.B) * a.kv_bstride, static_cast<uint64_t>(a.H) * DVP, a.ldv * 2, 64, DVP);
   if (rc) return rc;
   dim3 grid((p.Nq + kBQ - 1) / kBQ, a.H, a.B);
+  g_att_last = KL ? (BKV == 64 ? kAttKeylen64 : kAttKeylen128)
+                  : (DK == 192 ? kAttD160 : (DK == 128 ? kAttD80 : (BKV == 128 ? kAttCols128 : (SB == 2 ? kAttCols64Dbuf : kAttCols64ThreeCta))));
   VDB_CUDA_CHECK(launch_pdl(kernel, grid, dim3(64 + 128 * SW), smem, stream, p));
   count_launch();
   return VDB_OK;
@@ -937,6 +944,7 @@ static int launch_attention_fa(AttnParams& p, const AttnArgs& a, cudaStream_t st
                     ONES ? p.dv : DVP);          // ONES: the box leaves the static padding rows of the stage alone
   if (rc) return rc;
   dim3 grid((p.Nq + 2 * kBQ - 1) / (2 * kBQ), a.H, a.B);
+  g_att_last = kAttTwoTile;
   VDB_CUDA_CHECK(launch_pdl(kernel, grid, dim3(384), smem, stream, p));
   count_launch();
   return VDB_OK;
@@ -981,9 +989,14 @@ extern "C" {
 
 // debug aid (not part of the product ABI; stamps exist only in a -DVDB_TIMELINE build): 16 x 16 u64 device buffer
 void vdb_debug_attention_timeline(void* buf) { g_att_timeline = reinterpret_cast<unsigned long long*>(buf); }
+// debug aid (host side, not part of the product ABI): kernel family of the last attention launch on this thread —
+// 1 two-tile, 2 64-column double-buffered, 3 64-column three-CTA, 4 128-column, 5 d_head 65..80, 6 d_head 81..160,
+// 7 key-length 64-column, 8 key-length 128-column; 0 before the first launch
+int vdb_debug_attention_last(void) { return g_att_last; }
 
-// Padded head sizes the projection GEMMs must produce for a given d_head (see include/vdb200.h).
-int vdb_attention_dk_pad(int d_head) { return d_head <= 64 ? 64 : (d_head <= 128 ? 128 : (d_head <= 192 ? 192 : -1)); }
+// Padded head sizes the projection GEMMs must produce for a given d_head (see include/vdb200.h): one (DK, DVP) pair per
+// instantiated kernel, (64, 48 | 64), (128, 80) and (192, 160); d_head 81..160 all run on the last one.
+int vdb_attention_dk_pad(int d_head) { return d_head <= 64 ? 64 : (d_head <= 80 ? 128 : (d_head <= 160 ? 192 : -1)); }
 int vdb_attention_dv_pad(int d_head) {
   if (d_head <= 48) return 48;
   if (d_head <= 64) return 64;

@@ -964,6 +964,8 @@ static int pick_bn(int N, int act, int forced) {
 
 static unsigned long long* g_timeline = nullptr;
 static long long g_pair_launches = 0;
+// debug aid: {epilogue mode, BN, ksplit, CTA pair} of the last launch on this thread (vdb_debug_igemm_last)
+static thread_local int g_igemm_last[4] = {-1, 0, 0, 0};
 
 struct IgemmEpilogue {
   const float* bias = nullptr;
@@ -1137,6 +1139,7 @@ static int run_igemm(IgemmParams& p, const void* Wt, long long N, long long Ktot
     if (ln_in && mode == 4 && e.ln_on_cols) return set_error(VDB_ERR_UNSUPPORTED, "igemm: GEGLU with column statistics");
     mode = st_out ? 7 : mode + 2;
   }
+  g_igemm_last[0] = mode; g_igemm_last[1] = BN; g_igemm_last[2] = p.ksplit; g_igemm_last[3] = pair ? 1 : 0;
   if (pair && mode == 3) {
     ++g_pair_launches;                 // CTA pairs with the TMA-store epilogue (each CTA stores its own 128 rows)
     switch (BN) {
@@ -1235,6 +1238,9 @@ extern "C" {
 void vdb_debug_igemm_timeline(void* buf) { g_timeline = reinterpret_cast<unsigned long long*>(buf); }
 // debug aid: how many igemm launches ran as CTA pairs (cta_group::2)
 long long vdb_debug_pair_launches(void) { return g_pair_launches; }
+// debug aid (host side): out4 = {epilogue mode after the TMA-store / LayerNorm promotion (0..7), BN, ksplit, CTA pair 0/1} of the
+// last vdb_gemm_bf16 / vdb_gemm_ln_bf16 / vdb_conv3x3_bf16 launch on the calling thread ({-1, 0, 0, 0} before the first one)
+void vdb_debug_igemm_last(int* out4) { for (int i = 0; i < 4; ++i) out4[i] = g_igemm_last[i]; }
 
 // out[M,N] = act(alpha * ([A | A2] @ W^T + bias)) + resid     (see include/vdb200.h)
 int vdb_gemm_bf16(const void* A, long long M, long long K, long long lda, const void* A2, long long K2,
